@@ -6,6 +6,7 @@
         --master-port P bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...   # the reference's CPU path (gloo DDP on host cores)
     python bench.py --impl nccl ...        # comparator: stock torch DDP over NCCL (not the product)
+    python bench.py ... --dump-outputs DIR # also write what the last timed step computed (.npy)
 
 One step = forward + backward + Adam update of torchvision ResNet-50 (random init, synthetic
 224x224 batch, bf16 autocast, per-GPU batch 32 as in release/train_tests/benchmark/config.py:15),
@@ -53,8 +54,15 @@ def parse_args():
     p.add_argument("--no-nccl-comparator", action="store_true", help="skip the in-line NCCL comparator leg (N>1)")
     p.add_argument("--profile", action="store_true",
                    help="under ncu: skip the end-to-end and sweep legs (numbers printed in this mode are not bench values)")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="after the timed steps, write what the last one computed as DIR/<name>.npy (GPU arms)")
     p.add_argument("--cpu-worker", default=None, help=argparse.SUPPRESS)
-    return p.parse_args()
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        p.error("--dump-outputs applies to the GPU arms")
+    return args
 
 
 def env_rank():
@@ -134,6 +142,28 @@ def train_step(model, opt, x, y, device_type):
     return loss
 
 
+DUMP_PARAMS = 1 << 22  # parameters sampled by --dump-outputs: 16 MiB of the model's ~100 MiB
+
+
+def dump_outputs(out_dir, model, loss):
+    """Writes what one training step hands back: its loss (loss.npy), the updated parameters
+    (params.npy: the same seeded sample of DUMP_PARAMS positions of all parameters flattened in
+    model order, every run) and the BatchNorm running statistics (buffers.npy: every
+    floating-point buffer, flattened).  float32."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    with torch.no_grad():
+        flat = torch.cat([p.detach().reshape(-1).float() for p in model.parameters()])
+        pick = np.random.default_rng(0).choice(flat.numel(), min(DUMP_PARAMS, flat.numel()), replace=False)
+        params = flat[torch.from_numpy(np.sort(pick)).to(flat.device)].cpu().numpy()
+        buffers = torch.cat([b.detach().reshape(-1).float() for b in model.buffers() if b.is_floating_point()])
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().reshape(1).cpu().numpy())
+    np.save(os.path.join(out_dir, "params.npy"), params)
+    np.save(os.path.join(out_dir, "buffers.npy"), buffers.cpu().numpy())
+
+
 # ----------------------------------------------------------------------------- GPU arms
 def run_gpu(args):
     import torch
@@ -181,6 +211,7 @@ def run_gpu(args):
     dev_x = host_x.to(device)
     dev_y = host_y.to(device)
     loss_host = torch.zeros((), dtype=torch.float32).pin_memory()
+    last = {}  # loss of the most recent timed step, for --dump-outputs
 
     def timed(region_steps, resident: bool):
         """Returns ms for `region_steps` steps (device time, this rank)."""
@@ -201,6 +232,7 @@ def run_gpu(args):
                 loss_host.copy_(loss.detach().float(), non_blocking=True)
         t1.record()
         torch.cuda.synchronize()
+        last["loss"] = loss
         if world > 1:
             dist.barrier()
         torch.cuda.synchronize()
@@ -245,6 +277,9 @@ def run_gpu(args):
         for _ in range(2):
             timed(1, resident=False)
         ms_e2e = max_over_ranks(timed(args.steps, resident=False))
+    if args.dump_outputs and rank == 0:  # DDP keeps every replica identical
+        dump_outputs(args.dump_outputs, model.module, last["loss"])
+        log(f"outputs of the last timed step written to {args.dump_outputs}")
 
     global_batch = B * world
     value = global_batch * args.steps / (ms / 1e3)

@@ -314,6 +314,10 @@ static size_t oneshot_limit(const b200_comm *c) {
   return (size_t(5) << 19) / size_t(c->world);  // 2.5 MiB / n
 }
 
+const void *allreduce_module_kernel() {
+  return reinterpret_cast<const void *>(allreduce_ll_kernel<float, B200_SUM>);
+}
+
 }  // namespace b200
 
 using namespace b200;

@@ -1041,6 +1041,8 @@ int selftest_pipe_geometry(size_t nbytes, size_t chunk_bytes, int copy_ctas, int
   return B200_OK;
 }
 
+const void *allreduce_pipe_module_kernel() { return reinterpret_cast<const void *>(allgather_pull_kernel); }
+
 }  // namespace b200
 
 extern "C" int b200_selftest_pipe_geometry(size_t nbytes, size_t chunk_bytes, int copy_ctas, int world, int red_ctas,

@@ -21,6 +21,7 @@
 #include <chrono>
 #include <cstring>
 #include <map>
+#include <set>
 
 #include "comm.h"
 
@@ -65,8 +66,13 @@ struct Driver {
   CUresult (*MulticastUnbind)(CUmemGenericAllocationHandle, CUdevice, size_t, size_t) = nullptr;
   CUresult (*MulticastGetGranularity)(size_t *, const CUmulticastObjectProp *,
                                       CUmulticastGranularity_flags) = nullptr;
+  CUresult (*FuncGetModule)(CUmodule *, CUfunction) = nullptr;
+  CUresult (*ModuleGetFunctionCount)(unsigned int *, CUmodule) = nullptr;
+  CUresult (*ModuleEnumerateFunctions)(CUfunction *, unsigned int, CUmodule) = nullptr;
+  CUresult (*FuncLoad)(CUfunction) = nullptr;
   bool ok = false;
   bool has_multicast = false;
+  bool has_func_load = false;
 };
 
 template <typename F>
@@ -109,6 +115,12 @@ static Driver &driver() {
     mc &= load_sym("cuMulticastUnbind", &d.MulticastUnbind);
     mc &= load_sym("cuMulticastGetGranularity", &d.MulticastGetGranularity);
     d.has_multicast = mc;
+    bool fl = true;
+    fl &= load_sym("cuFuncGetModule", &d.FuncGetModule);
+    fl &= load_sym("cuModuleGetFunctionCount", &d.ModuleGetFunctionCount);
+    fl &= load_sym("cuModuleEnumerateFunctions", &d.ModuleEnumerateFunctions);
+    fl &= load_sym("cuFuncLoad", &d.FuncLoad);
+    d.has_func_load = fl;
   });
   return d;
 }
@@ -471,6 +483,37 @@ int check_usable(b200_comm *c) {
   return B200_OK;
 }
 
+// CUDA loads kernels lazily by default, and loading a kernel at its first launch may synchronise the
+// context.  The collective kernels spin until their peers' kernels run, so where ranks share a context
+// (several ranks on one GPU, thread actors of one process) a first launch can wait for a kernel that
+// is itself waiting for that launch, until the device watchdog gives up.  Every kernel of the library
+// is therefore loaded on a device before the first communicator there can launch anything.
+static int preload_kernels(int device) {
+  static std::mutex mu;
+  static std::set<int> done;
+  std::lock_guard<std::mutex> lk(mu);
+  if (done.count(device)) return B200_OK;
+  Driver &d = driver();
+  if (!d.has_func_load) {
+    set_error("CUDA driver lacks cuModuleEnumerateFunctions / cuFuncLoad (needs CUDA 12.4 or newer)");
+    return B200_ERR_UNSUPPORTED;
+  }
+  for (const void *k : {allreduce_module_kernel(), allreduce_pipe_module_kernel(), copy_ops_module_kernel(),
+                        grad_module_kernel(), p2p_module_kernel(), reduce_ops_module_kernel()}) {
+    cudaFunction_t f = nullptr;
+    B200_CHECK_CUDA(cudaGetFuncBySymbol(&f, k));
+    CUmodule mod = nullptr;
+    B200_CHECK_CU(d.FuncGetModule(&mod, f));
+    unsigned int n = 0;
+    B200_CHECK_CU(d.ModuleGetFunctionCount(&n, mod));
+    std::vector<CUfunction> fns(n);
+    B200_CHECK_CU(d.ModuleEnumerateFunctions(fns.data(), n, mod));
+    for (CUfunction fn : fns) B200_CHECK_CU(d.FuncLoad(fn));
+  }
+  done.insert(device);
+  return B200_OK;
+}
+
 }  // namespace b200
 
 using namespace b200;
@@ -527,6 +570,8 @@ int b200_comm_create(int world_size, int rank, int device, const b200_config_t *
     set_error("CUDA driver lacks the virtual memory management API");
     return B200_ERR_UNSUPPORTED;
   }
+  const int pre = preload_kernels(device);
+  if (pre) return pre;
 
   b200_comm *c = new b200_comm();
   c->world = world_size;

@@ -90,4 +90,13 @@ namespace b200 {
 // implemented in bootstrap.cu
 int check_usable(b200_comm *c);
 inline size_t round_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
+
+// One kernel of every translation unit that defines kernels (each is a module of its own in the
+// shared object): b200_comm_create loads every function of these modules up front.
+const void *allreduce_module_kernel();
+const void *allreduce_pipe_module_kernel();
+const void *copy_ops_module_kernel();
+const void *grad_module_kernel();
+const void *p2p_module_kernel();
+const void *reduce_ops_module_kernel();
 }  // namespace b200

@@ -105,6 +105,8 @@ __global__ void barrier_kernel(DevComm c) {
   finish_launch(c);
 }
 
+const void *copy_ops_module_kernel() { return reinterpret_cast<const void *>(barrier_kernel); }
+
 }  // namespace b200
 
 using namespace b200;

@@ -236,6 +236,8 @@ static int launch_grad(b200_comm *c, GradArgs a, cudaStream_t stream) {
   return B200_OK;
 }
 
+const void *grad_module_kernel() { return reinterpret_cast<const void *>(grad_local_scalar_kernel<float>); }
+
 }  // namespace b200
 
 using namespace b200;

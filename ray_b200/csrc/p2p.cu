@@ -297,6 +297,8 @@ static int p2p_common(b200_comm *c, void *buf, size_t nbytes, int peer, cudaStre
   return B200_OK;
 }
 
+const void *p2p_module_kernel() { return reinterpret_cast<const void *>(get_ldst_kernel); }
+
 }  // namespace b200
 
 using namespace b200;

@@ -137,6 +137,10 @@ static int launch_reduce(b200_comm *c, const ReduceArgs &a, cudaStream_t stream)
   return B200_OK;
 }
 
+const void *reduce_ops_module_kernel() {
+  return reinterpret_cast<const void *>(reducescatter_kernel<float, B200_SUM>);
+}
+
 }  // namespace b200
 
 using namespace b200;

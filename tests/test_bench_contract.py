@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -35,10 +37,31 @@ def test_reference_arm_non_zero_ranks_exit_quietly():
     assert out.returncode == 0 and out.stdout.strip() == ""
 
 
+@pytest.mark.parametrize("extra", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "out"]])
+def test_bad_arguments_are_refused(extra):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True,
+                         timeout=120)
+    assert out.returncode == 2 and out.stdout.strip() == "", out.stderr[-2000:]
+
+
+@pytest.mark.gpu
+def test_gpu_arm_dumps_the_last_timed_step(tmp_path):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1",
+                          "--no-cpu-baseline", "--dump-outputs", str(tmp_path)], capture_output=True, text=True,
+                         timeout=900)
+    assert out.returncode == 0, out.stderr[-2000:]
+    lines = [l for l in out.stdout.splitlines() if l.strip()]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == 2
+    files = {p.name: p for p in tmp_path.iterdir()}
+    assert set(files) == {"loss.npy", "params.npy", "buffers.npy"}
+    assert sum(p.stat().st_size for p in files.values()) <= 64 << 20
+    for p in files.values():
+        a = np.load(p)
+        assert a.dtype == np.float32 and a.size > 0 and np.isfinite(a).all(), p.name
+
+
 def test_gpu_arm_fails_loudly_without_a_gpu():
     if torch.cuda.is_available():
-        import pytest
-
         pytest.skip("GPU present")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "1", "--warmup", "1"],
                          capture_output=True, text=True, timeout=300)

@@ -78,6 +78,9 @@ class Actors:
         for e in err:
             if e is not None:
                 raise e
+        for c in self.comms:  # a kernel that gave up (watchdog) leaves its output unwritten
+            if c.comm is not None and not c.comm.closed:
+                c.comm.check_status()
         return out
 
     def dev(self, r):
