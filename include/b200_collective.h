@@ -82,7 +82,7 @@ typedef enum {
   B200_ALGO_NVLS = 3,     /* multimem.ld_reduce + multimem.st through the NVSwitch */
   B200_ALGO_LL = 4,       /* flag-in-data push, no barrier (<= 64 KiB) */
   B200_ALGO_PIPE = 5      /* chunk-pipelined: TMA copy-in | reduce | TMA copy-out roles in one launch
-                             (n == 2: one-shot push straight into the peer's slot) */
+                             (n == 2: TMA copy-in | bulk-load the peer's slot and reduce into the output) */
 } b200_algo_t;
 
 typedef struct {
@@ -239,16 +239,13 @@ typedef enum {
   B200_PARAM_NVLS_CTAS = 2,         /* CTAs of the NVSwitch reduce phase: zero-copy default 64, staged default all */
   B200_PARAM_LL_MAX_BYTES = 3,      /* all-reduce messages up to this size use the LL kernel (default 32 KiB / 2 ranks ... 4 KiB / 8 ranks) */
   B200_PARAM_PIPE_MIN_BYTES = 4,    /* AUTO uses the pipelined kernels from this size on (ordinary, 16-byte aligned tensors) */
-  B200_PARAM_PIPE_CHUNK_BYTES = 5,  /* pipeline chunk size (default 1 MiB; rounded up to 1 MiB multiples) */
-  B200_PARAM_PIPE_COPY_CTAS = 6,    /* CTAs per TMA copy role (power of two; default 8, push 16) */
-  B200_PARAM_PIPE_RED_CTAS = 7,     /* CTAs of the reduce role (default 48) */
-  B200_PARAM_PIPE_VARIANT = 8,      /* B200_ALGO_PIPE only: force 0 = push, 1 = NVLS roles, 2 = peer ld/st roles, 3 = pull (2 ranks) */
-  B200_PARAM_GRAD_LOCAL_UNROLL = 9, /* world 1 gradient kernel: 16-byte wire units per thread (1, 2, 4, 8) */
-  B200_PARAM_P2P_BULK_MIN_CHUNK = 10, /* send/recv: chunks from this size on move with the TMA bulk-copy kernel (0 = never; default 32 KiB) */
-  B200_PARAM_BULK_CFG = 11,         /* send: bulk-engine (lookahead, completion lag) flavour, tuning experiments only */
-  B200_PARAM_AG_PULL_MIN_BYTES = 12, /* all-gather: per-rank size from which the pull kernel is used (0 = never; default 4 MiB) */
-  B200_PARAM_PIPE_RING = 13,        /* n >= 3 pipeline: 0 = split messages larger than the staging slot into several launches; default: one launch, the slot is a ring of chunks */
-  B200_PARAM_COUNT = 14
+  B200_PARAM_PIPE_CHUNK_BYTES = 5,  /* pipeline chunk size, rounded up to 1 MiB multiples (all-reduce default 1 MiB at 2 ranks, 4 MiB at <= 4, 8 MiB above; pull all-gather 1 MiB) */
+  B200_PARAM_PIPE_COPY_CTAS = 6,    /* CTAs per TMA copy role (power of two; default 32 for the 2-rank pull all-reduce, 16 otherwise) */
+  B200_PARAM_PIPE_RED_CTAS = 7,     /* CTAs of the reduce / pull role (all-reduce default 32 for the 2-rank pull kernel, 64 at <= 4 ranks, 32 above; pull all-gather 64 at 2 ranks, 48 at <= 4, 32 above) */
+  B200_PARAM_PIPE_VARIANT = 8,      /* B200_ALGO_PIPE only: force 1 = NVLS roles, 2 = peer ld/st roles, 3 = pull (2 ranks); other values are rejected */
+  B200_PARAM_P2P_BULK_MIN_CHUNK = 9, /* send/recv: chunks from this size on move with the TMA bulk-copy kernel (0 = never; default 32 KiB) */
+  B200_PARAM_AG_PULL_MIN_BYTES = 10, /* all-gather: per-rank size from which the pull kernel is used (0 = never; default 4 MiB) */
+  B200_PARAM_COUNT = 11
 } b200_param_t;
 int b200_comm_set_param(b200_comm_t comm, int param, long long value);
 

@@ -32,8 +32,7 @@ SUM, PROD, MIN, MAX, AVG = range(5)
 # tuning parameters (b200_param_t)
 (PARAM_ONESHOT_MAX_BYTES, PARAM_NVLS_MIN_WORLD, PARAM_NVLS_CTAS, PARAM_LL_MAX_BYTES, PARAM_PIPE_MIN_BYTES,
  PARAM_PIPE_CHUNK_BYTES, PARAM_PIPE_COPY_CTAS, PARAM_PIPE_RED_CTAS, PARAM_PIPE_VARIANT,
- PARAM_GRAD_LOCAL_UNROLL, PARAM_P2P_BULK_MIN_CHUNK, PARAM_BULK_CFG, PARAM_AG_PULL_MIN_BYTES,
- PARAM_PIPE_RING) = range(14)
+ PARAM_P2P_BULK_MIN_CHUNK, PARAM_AG_PULL_MIN_BYTES) = range(11)
 # algorithms (b200_algo_t)
 ALGO_AUTO, ALGO_ONESHOT, ALGO_TWOSHOT, ALGO_NVLS, ALGO_LL, ALGO_PIPE = range(6)
 

@@ -301,12 +301,7 @@ static size_t pipe_min_bytes(const b200_comm *c) {
 }
 
 static size_t oneshot_limit(const b200_comm *c) {
-  static long long env = [] {
-    const char *s = getenv("B200_ONESHOT_MAX_BYTES");
-    return s ? atoll(s) : -1ll;
-  }();
   if (c->params[B200_PARAM_ONESHOT_MAX_BYTES] >= 0) return size_t(c->params[B200_PARAM_ONESHOT_MAX_BYTES]);
-  if (env >= 0) return size_t(env);
   // each rank reads world * nbytes in the one-shot scheme.  Break-even against the two-shot kernel
   // (profiles/r01 sweeps: 2 ranks ~1 MiB, 8 ranks ~256 KiB; profiles/r02/bench_n4: 256 KiB one-shot
   // 16 us, 1 MiB two-shot 24 us); the 0.5 MB PPO gradient vector of BASELINE configs[3] falls on
@@ -369,7 +364,7 @@ extern "C" int b200_allreduce(b200_comm_t c, const void *in, void *out, size_t c
   // the two staging passes with the NVLink phase (allreduce_pipe.cu).  They move whole 16-byte
   // units with the bulk-copy engine, so they need aligned operands.
   int pipe_variant = -1;
-  if (sym_off < 0 && is_aligned16(in) && is_aligned16(out) && (total & 15) == 0 && pipe_max_bytes(c, 0) > 0 &&
+  if (sym_off < 0 && is_aligned16(in) && is_aligned16(out) && (total & 15) == 0 && pipe_chunk_bytes(c) > 0 &&
       (algo == B200_ALGO_PIPE || (algo == B200_ALGO_AUTO && total >= pipe_min_bytes(c)))) {
     if (c->world == 2) pipe_variant = PIPE_PULL;
     else if (c->mc_active && nvls_capable(dtype, op)) pipe_variant = PIPE_NVLS;

@@ -14,12 +14,6 @@
 //                                                                              -> flag1[k][rank]
 //     copy-out CTAs : wait flag1[k][*]; own slot -> user tensor, TMA bulk copies
 //
-//   allreduce_push_kernel (n == 2: one-shot push, the link carries S per direction either way)
-//     push     CTAs : user tensor -> the PEER's slot over NVLink, TMA bulk copies (the stage-in
-//                     pass and the transfer are the same bytes)                -> flag0[k][rank]
-//     reduce   CTAs : wait flag0[k][*]; out = user (op) slot, rank-ascending, straight into the
-//                     caller's tensor -- no stage-out pass at all
-//
 // A copy role is one thread driving the bulk-copy unit (bulk_copy.cuh), so it costs a few CTAs;
 // the reduce roles are ordinary 512-thread CTAs with 16-byte accesses.
 //
@@ -123,40 +117,12 @@ __device__ __forceinline__ bool chunk_arrive_fenced(uint32_t *cnt, uint32_t expe
   }
   return false;
 }
-__device__ __forceinline__ bool chunk_arrive(uint32_t *cnt, uint32_t expected) {
-  __threadfence_system();
-  return chunk_arrive_fenced(cnt, expected);
-}
 __device__ __forceinline__ void signal_all(const DevComm &c, size_t flag_word, uint32_t value) {
   for (int i = 0; i < c.world; ++i) {
     int p = c.rank + i;  // own pad first (local consumers), then walk the peers
     if (p >= c.world) p -= c.world;
     st_relaxed_sys(c.sig[p] + flag_word + c.rank, value);
   }
-}
-// All threads: wait until every rank's flag of chunk k reached `value`.
-__device__ __forceinline__ bool cta_wait_chunk(const DevComm &c, size_t flag_base, uint32_t k, uint32_t value) {
-  __shared__ int ok_flag;
-  if (threadIdx.x == 0) ok_flag = 1;
-  __syncthreads();
-  if (threadIdx.x < c.world) {
-    if (!wait_flag_ge(c, c.sig[c.rank] + flag_base + size_t(k) * kMaxRanks + threadIdx.x, value)) ok_flag = 0;
-  }
-  __syncthreads();
-  return ok_flag != 0;
-}
-// One thread (the bulk-copy driver): same test, optionally non-blocking.
-__device__ __forceinline__ int thread_wait_chunk(const DevComm &c, size_t flag_base, uint32_t k, uint32_t value,
-                                                 bool block) {
-  const uint32_t *f = c.sig[c.rank] + flag_base + size_t(k) * kMaxRanks;
-  for (int p = 0; p < c.world; ++p) {
-    if (block) {
-      if (!wait_flag_ge(c, f + p, value)) return -1;
-    } else if (int32_t(ld_acquire_sys(f + p) - value) < 0) {
-      return 0;
-    }
-  }
-  return 1;
 }
 
 // Scout thread: the consumers of a chunk flag (copy-out, pull) must not pay for the flag wait in
@@ -192,7 +158,7 @@ __device__ __forceinline__ int scout_gate(ChunkScout *sc, uint32_t k, bool block
   return 1;
 }
 
-// Flag thread of a copy-in / push CTA: publish flag0 of every chunk this CTA finished.
+// Flag thread of a copy-in CTA: publish flag0 of every chunk this CTA finished.
 __device__ __forceinline__ void copy_flag_thread(const DevComm &c, const PipeGeom &g, CopyMailbox *mb,
                                                  uint32_t nchunks, uint32_t value) {
   uint32_t published = 0;
@@ -295,8 +261,6 @@ struct ItemIter {
     }
     return false;
   }
-  // the scout only has to follow the chunks up to the last one this CTA works on
-  __host__ __device__ uint32_t last_chunk_needed() const { return g.K; }
 };
 
 // ---------------------------------------------------------------------------
@@ -334,7 +298,7 @@ __global__ void __launch_bounds__(kThreads + 32, 1) allreduce_pipe_kernel(DevCom
     ItemIter iter(g, r, n, uint32_t(b - G), uint32_t(Gr));
     if (threadIdx.x >= kThreads) {
       if (threadIdx.x == kThreads) {
-        scout_thread(c, kSigPipe0, ep + 1, iter.last_chunk_needed(), &sc);
+        scout_thread(c, kSigPipe0, ep + 1, g.K, &sc);
       } else if (threadIdx.x == kThreads + 1) {
         uint32_t published = 0, k = 0;
         bool have = iter.next(k);
@@ -457,111 +421,6 @@ __global__ void __launch_bounds__(kThreads + 32, 1) allreduce_pipe_kernel(DevCom
           });
     } else if (threadIdx.x == 32) {
       scout_thread(c, kSigPipe1, ep + 2, my_chunks, &sc);
-    }
-  }
-  finish_launch(c);
-}
-
-// ---------------------------------------------------------------------------
-// one-shot push, n == 2 (kept for comparison with the pull kernel below, which replaced it as the default)
-// ---------------------------------------------------------------------------
-template <typename T, int OP, int UNR, int NW>  // NW: compile-time bound on the world size
-__device__ __forceinline__ void push_reduce_item(const DevComm &c, const PipeArgs &a, size_t sub, size_t off,
-                                                 size_t ubase, size_t u0, size_t uend) {
-  using Tr = Traits<T>;
-  const int n = c.world, r = c.rank;
-  const char *slot = c.data[r] + off;
-  uint4 v[UNR][NW];
-#pragma unroll
-  for (int q = 0; q < UNR; ++q) {
-    const size_t u = u0 + size_t(q) * kThreads;
-    if (u < uend) {
-      const size_t byte = (ubase + u) << 4;
-#pragma unroll
-      for (int p = 0; p < NW; ++p) {
-        if (p < n) {
-          if (p == r) v[q][p] = ld_stream(a.in + byte);
-          else v[q][p] = ld_peer(slot + size_t(p < r ? p : p - 1) * sub + byte);
-        }
-      }
-    }
-  }
-#pragma unroll
-  for (int q = 0; q < UNR; ++q) {
-    const size_t u = u0 + size_t(q) * kThreads;
-    if (u < uend) {
-      typename Tr::Acc acc = Tr::unpack(v[q][0]);
-#pragma unroll
-      for (int p = 1; p < NW; ++p)
-        if (p < n) Tr::template reduce<OP>(acc, Tr::unpack(v[q][p]));  // rank-ascending
-      if (OP == B200_AVG) Tr::average(acc, n);
-      st_vec(a.out + ((ubase + u) << 4), Tr::pack(acc));
-    }
-  }
-}
-
-template <typename T, int OP>
-__global__ void __launch_bounds__(kThreads, 1) allreduce_push_kernel(DevComm c, PipeArgs a) {
-  extern __shared__ __align__(128) char dyn_smem[];
-  const uint32_t launch = c.st->launch_ctr;
-  const uint32_t ep = launch * 4u;
-  const size_t off = staging_slot_offset(launch, a.staging_bytes);
-  const PipeGeom g = make_geom(a);
-  const int n = c.world, r = c.rank;
-  const int G = int(g.G), Gr = int(gridDim.x) - G;
-  const int b = blockIdx.x;
-  const size_t sub = g.S;  // the peer's data starts at the slot base (2 ranks: one sub-slot)
-
-  if (b < G) {
-    // ---- push: my tensor into the peer's slot ---------------------------------------------------
-    __shared__ CopyMailbox mb;
-    if (threadIdx.x == 0) {
-      mb.chunks_done = 0;
-      mb.stop = 0;
-    }
-    const BulkRing ring = bulk_ring_init(dyn_smem);
-    const uint32_t j = uint32_t(b);
-    const uint32_t my_chunks = chunks_of_cta(g, j);
-    if (threadIdx.x == 0) {
-      char *peer_slot = c.data[1 - r] + off;
-      const bool ok = bulk_copy_segments<BulkRemote>(
-          ring, my_chunks,
-          [&](uint32_t k) {
-            const size_t o = share_off(g, j, k);
-            return BulkSeg{a.in + o, peer_slot + o, share_len(g, j, k)};
-          },
-          [&](uint32_t, bool) { return 1; }, [&](uint32_t k) { mailbox_post(&mb, k + 1); });
-      if (!ok) mb.stop = 1;
-    } else if (threadIdx.x == 32) {
-      copy_flag_thread(c, g, &mb, my_chunks, ep + 1);
-    }
-  } else {
-    // ---- reduce: own tensor (op) what the peers pushed, straight into the caller's tensor ---
-    const int me = b - G;
-    size_t item_base = 0;
-    for (uint32_t k = 0; k < g.K; ++k) {
-      const size_t cu = chunk_len(g, k) >> 4;
-      const size_t nitems = (cu + kItemUnits - 1) / kItemUnits;
-      size_t it = (size_t(me) + size_t(Gr) - item_base % size_t(Gr)) % size_t(Gr);
-      item_base += nitems;
-      if (it >= nitems) continue;
-      // flag0[k][p] for p != r: p's chunk has landed here; p == r: the local push CTAs are done
-      // READING chunk k of the caller's tensor, so it may be overwritten in place.
-      if (threadIdx.x == 0) trace_event(c, 20, k);
-      if (!cta_wait_chunk(c, kSigPipe0, k, ep + 1)) break;
-      if (threadIdx.x == 0) trace_event(c, 21, k);
-      const size_t ubase = (size_t(k) * g.C) >> 4;
-      for (; it < nitems; it += size_t(Gr)) {
-        const size_t u0 = it * kItemUnits + threadIdx.x;
-        if (n == 2) {
-          push_reduce_item<T, OP, 4, 2>(c, a, sub, off, ubase, u0, cu);
-        } else {
-#pragma unroll 1
-          for (int q = 0; q < kItemUnroll; ++q)
-            push_reduce_item<T, OP, 1, kMaxRanks>(c, a, sub, off, ubase, u0 + size_t(q) * kThreads, cu);
-        }
-        if (threadIdx.x == 0) trace_event(c, 22, k);
-      }
     }
   }
   finish_launch(c);
@@ -827,10 +686,10 @@ size_t pipe_chunk_bytes(const b200_comm *c) {
   return C < fit ? C : fit;                                 // 0: slot too small for the pipeline
 }
 
-// chunk ring of the n >= 3 pipeline (B200_PARAM_PIPE_RING: 0 disables it)
+// chunk ring of the n >= 3 pipeline, used whenever the slot holds at least 4 chunks: one launch
+// beat splitting the message into launches in every measured case (profiles/r02/ring_check.log)
 static bool pipe_ring_enabled(const b200_comm *c, int variant) {
   if (variant != PIPE_NVLS && variant != PIPE_PEER) return false;  // pull kernels: the READER is a peer
-  if (c->params[B200_PARAM_PIPE_RING] == 0) return false;
   const size_t C = pipe_chunk_bytes(c);
   return C && c->staging_bytes / C >= 4;
 }
@@ -853,8 +712,8 @@ int launch_allreduce_pipe(b200_comm *c, const char *in, char *out, size_t nbytes
   const long long pc = c->params[B200_PARAM_PIPE_COPY_CTAS];
   const long long pr = c->params[B200_PARAM_PIPE_RED_CTAS];
   int G = pc > 0 ? int(pc) : (variant == PIPE_PULL ? 32 : 16);
-  int Gr = pr > 0 ? int(pr) : (variant == PIPE_PULL ? 32 : (variant == PIPE_PUSH ? 64 : (c->world <= 4 ? 64 : 32)));
-  const int roles = (variant == PIPE_PUSH || variant == PIPE_PULL) ? 1 : 2;
+  int Gr = pr > 0 ? int(pr) : (variant == PIPE_PULL ? 32 : (c->world <= 4 ? 64 : 32));
+  const int roles = variant == PIPE_PULL ? 1 : 2;
   int cap = c->forced_blocks > 0 ? c->forced_blocks : c->sm_count;
   if (roles * G + Gr > cap) {  // shared-GPU harness / small parts: shrink, keep at least one reducer
     while (G > 1 && roles * G + 1 > cap / 2) G /= 2;
@@ -877,14 +736,6 @@ int launch_allreduce_pipe(b200_comm *c, const char *in, char *out, size_t nbytes
     auto k = allreduce_pull_kernel<T, OP>;
     if ((rc = set_dyn_smem(c->device, reinterpret_cast<const void *>(k)))) return rc;
     k<<<grid, kThreads + 32, kBulkSmemBytes, stream>>>(dc, a);  // + one service warp (scout)
-  } else if (variant == PIPE_PUSH) {
-    if (c->world != 2) {
-      set_error("the push all-reduce is a 2-rank kernel");
-      return B200_ERR_UNSUPPORTED;
-    }
-    auto k = allreduce_push_kernel<T, OP>;
-    if ((rc = set_dyn_smem(c->device, reinterpret_cast<const void *>(k)))) return rc;
-    k<<<grid, kThreads, kBulkSmemBytes, stream>>>(dc, a);
   } else if (variant == PIPE_NVLS) {
     if constexpr (Multimem<T>::kSum && (OP == B200_SUM || OP == B200_AVG)) {
       auto k = allreduce_pipe_kernel<T, OP, true>;

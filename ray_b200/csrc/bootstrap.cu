@@ -24,6 +24,7 @@
 #include <set>
 
 #include "comm.h"
+#include "pipe.h"
 
 namespace b200 {
 
@@ -995,7 +996,7 @@ void b200_pool_free(void *ptr, size_t size, int device, void *stream) {
 }
 
 const char *b200_last_error(void) { return g_err; }
-const char *b200_version(void) { return "b200_collective 0.2 (sm_100a)"; }
+const char *b200_version(void) { return "b200_collective 0.3 (sm_100a)"; }
 
 size_t b200_dtype_size(int dtype) {
   switch (dtype) {
@@ -1058,6 +1059,11 @@ int b200_comm_trace_read(b200_comm_t c, unsigned long long *out, unsigned int ma
 int b200_comm_set_param(b200_comm_t c, int param, long long value) {
   if (!c || param < 0 || param >= B200_PARAM_COUNT) {
     set_error("unknown parameter %d", param);
+    return B200_ERR_INVALID;
+  }
+  if (param == B200_PARAM_PIPE_VARIANT && value != -1 && value != PIPE_NVLS && value != PIPE_PEER && value != PIPE_PULL) {
+    set_error("B200_PARAM_PIPE_VARIANT must be -1, %d (NVLS), %d (peer) or %d (pull), got %lld", PIPE_NVLS, PIPE_PEER,
+              PIPE_PULL, value);
     return B200_ERR_INVALID;
   }
   c->params[param] = value;

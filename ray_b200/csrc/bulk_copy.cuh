@@ -44,10 +44,6 @@ struct BulkRemote {
 struct BulkPull {
   static constexpr int kLookahead = 5, kLag = kBulkLagLocal;
 };
-template <int LA, int LAG>
-struct BulkCfg {  // experiments
-  static constexpr int kLookahead = LA, kLag = LAG;
-};
 constexpr size_t kBulkSmemBytes = size_t(kBulkStages) * kBulkTile + 16 * kBulkStages;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) {

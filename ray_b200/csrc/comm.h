@@ -4,6 +4,7 @@
 #include <cuda.h>
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <array>
 #include <atomic>
 #include <cstdarg>
@@ -78,11 +79,12 @@ struct b200_comm {
 
   std::atomic<uint64_t> launches{0};
   int forced_blocks = 0;
-  long long params[B200_PARAM_COUNT] = {-1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1, -1};
+  long long params[B200_PARAM_COUNT];  // b200_comm_set_param values; -1 = default
   int sm_count = 148;
   std::atomic<bool> aborted{false};
   std::mutex mu;
 
+  b200_comm() { std::fill(std::begin(params), std::end(params), -1ll); }
   b200::DevComm dev() const;
 };
 

@@ -143,10 +143,10 @@ extern "C" int b200_allgather(b200_comm_t c, const void *in, void *const *outs, 
   {
     const long long pm = c->params[B200_PARAM_AG_PULL_MIN_BYTES];
     const size_t pull_min = pm >= 0 ? size_t(pm) : (size_t(4) << 20);  // 4 ranks: 1 MiB/rank 49 us pulled vs 28 us staged
-    bool aligned = is_aligned16(in) && (total & 15) == 0 && pm != 0 && pipe_max_bytes(c, 0) > 0;
+    bool aligned = is_aligned16(in) && (total & 15) == 0 && pm != 0 && pipe_chunk_bytes(c) > 0;
     for (int p = 0; p < c->world; ++p) aligned = aligned && is_aligned16(outs[p]);
     if (aligned && total >= pull_min) {
-      const size_t cap = pipe_max_bytes(c, 0) / (size_t(1) << 20) * (size_t(1) << 20);
+      const size_t cap = pipe_max_bytes(c, PIPE_PULL) / (size_t(1) << 20) * (size_t(1) << 20);
       const size_t step = cap ? cap : c->staging_bytes;
       for (size_t done = 0; done < total;) {
         const size_t nbytes = (total - done) < step ? (total - done) : step;

@@ -141,12 +141,13 @@ __global__ void __launch_bounds__(kThreads, 1) grad_allreduce_kernel(DevComm c, 
 }
 
 // world == 1: the same arithmetic without any peer (scale, round-trip through the wire type).
-// Pure HBM streaming (8 B per element).  One-shot grid: every thread owns UNR wire units (all
-// loads issued before the first store) and the hardware CTA scheduler does the load balancing --
-// no flag rows are involved, so the grid is NOT clamped to kMaxBlocks (round-1 ran this kernel
-// at 43 % occupancy because of that clamp).
+// Pure HBM streaming (8 B per element).  One-shot grid: every thread owns one 16-byte unit and the
+// hardware CTA scheduler does the load balancing -- no flag rows are involved, so the grid is NOT
+// clamped to kMaxBlocks (round-1 ran this kernel at 43 % occupancy because of that clamp).  One
+// unit per thread was best or tied against 2, 4 and 8 at every bucket size and wire type
+// (profiles/r02/grad_local_sweep_events.txt, grad_local_sweep_ncu.txt).
 constexpr int kLocalThreads = 256;
-// One thread = UNR x 16 bytes of the fp32 bucket (4 elements), whatever the wire type: nothing is
+// One thread = 16 bytes of the fp32 bucket (4 elements), whatever the wire type: nothing is
 // stored in wire format here, so the 8-element wire units of the multi-rank kernels would only
 // halve the thread count (ncu, 60 MB bucket: 20.0 us with 8-element units, 15.1 us with 4).
 template <typename W>
@@ -163,22 +164,12 @@ __device__ __forceinline__ uint4 wire_round_trip(uint4 v, float scale) {
   return make_uint4(__float_as_uint(f[0]), __float_as_uint(f[1]), __float_as_uint(f[2]), __float_as_uint(f[3]));
 }
 
-template <typename W, int UNR>
+template <typename W>
 __global__ void __launch_bounds__(kLocalThreads) grad_local_kernel(GradArgs a) {
   const size_t U = a.count >> 2;  // whole 16-byte units; the host sends the ragged tail separately
-  const size_t u0 = size_t(blockIdx.x) * kLocalThreads * UNR + threadIdx.x;
+  const size_t u = size_t(blockIdx.x) * kLocalThreads + threadIdx.x;
   uint4 *g = reinterpret_cast<uint4 *>(a.grad);
-  uint4 w[UNR];
-#pragma unroll
-  for (int k = 0; k < UNR; ++k) {
-    const size_t u = u0 + size_t(k) * kLocalThreads;
-    if (u < U) w[k] = ld_stream(g + u);
-  }
-#pragma unroll
-  for (int k = 0; k < UNR; ++k) {
-    const size_t u = u0 + size_t(k) * kLocalThreads;
-    if (u < U) st_vec(g + u, wire_round_trip<W>(w[k], a.scale));
-  }
+  if (u < U) st_vec(g + u, wire_round_trip<W>(ld_stream(g + u), a.scale));
 }
 
 // unaligned buckets / the last count % 4 elements
@@ -192,15 +183,14 @@ __global__ void grad_local_scalar_kernel(GradArgs a) {
   }
 }
 
-template <typename W, int UNR>
+template <typename W>
 static void launch_grad_local(const GradArgs &a, cudaStream_t stream) {
   if (!is_aligned16(a.grad)) {
     grad_local_scalar_kernel<W><<<1184, 256, 0, stream>>>(a);
     return;
   }
   const size_t U = a.count >> 2;
-  const size_t per_cta = size_t(kLocalThreads) * UNR;
-  if (U) grad_local_kernel<W, UNR><<<unsigned((U + per_cta - 1) / per_cta), kLocalThreads, 0, stream>>>(a);
+  if (U) grad_local_kernel<W><<<unsigned((U + kLocalThreads - 1) / kLocalThreads), kLocalThreads, 0, stream>>>(a);
   if (a.count & 3) {
     GradArgs tail = a;
     tail.grad = a.grad + (U << 2);
@@ -214,14 +204,7 @@ static int launch_grad(b200_comm *c, GradArgs a, cudaStream_t stream) {
   constexpr int E = Wire<W>::kElems;
   const size_t U = (a.count + E - 1) / E;
   if (c->world == 1) {
-    // units per thread: tuning knob, default measured on B200 (profiles/r02/grad_local_sweep.txt)
-    const long long unr = c->params[B200_PARAM_GRAD_LOCAL_UNROLL];
-    switch (unr > 0 ? int(unr) : 1) {
-      case 2: launch_grad_local<W, 2>(a, stream); break;
-      case 4: launch_grad_local<W, 4>(a, stream); break;
-      case 8: launch_grad_local<W, 8>(a, stream); break;
-      default: launch_grad_local<W, 1>(a, stream); break;
-    }
+    launch_grad_local<W>(a, stream);
     B200_LAUNCH_CHECK(c);
     return B200_OK;
   }

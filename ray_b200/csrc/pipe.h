@@ -4,14 +4,15 @@
 
 namespace b200 {
 
+// values of B200_PARAM_PIPE_VARIANT
 enum PipeVariant {
-  PIPE_PUSH = 0,  // one-shot push into the peers' slots (kept for comparison; slower than PIPE_PULL)
   PIPE_NVLS = 1,  // copy-in | multimem.ld_reduce + multimem.st | copy-out
   PIPE_PEER = 2,  // copy-in | peer loads + peer stores         | copy-out
   PIPE_PULL = 3   // n == 2: copy-in | bulk-load the peer's slot + reduce into the caller's tensor
 };
 
-// chunk size C of the pipeline (B200_PARAM_PIPE_CHUNK_BYTES, default 1 MiB)
+// chunk size C of the pipeline (B200_PARAM_PIPE_CHUNK_BYTES; default 1 MiB at 2 ranks, 4 MiB at
+// <= 4, 8 MiB above); 0 when the staging slot is too small for the pipeline
 size_t pipe_chunk_bytes(const b200_comm *c);
 // largest message one launch can take (a multiple of C)
 size_t pipe_max_bytes(const b200_comm *c, int variant);

@@ -12,7 +12,7 @@ world = int(sys.argv[1]) if len(sys.argv) > 1 else 2
 g = LocalGroup(world, timeout_ms=10000, staging_bytes=40 << 20, inbox_bytes=2 << 20)
 print("multicast", g.has_multicast, "devices", g.devices)
 MiB = 1 << 20
-variants = [("peer", 2)] + ([("pull", 3), ("push", 0)] if world == 2 else []) + ([("nvls", 1)] if g.has_multicast else [])
+variants = [("peer", 2)] + ([("pull", 3)] if world == 2 else []) + ([("nvls", 1)] if g.has_multicast else [])
 for vname, v in variants:
     for c in g.comms:
         c.set_param(N.PARAM_PIPE_VARIANT, v)

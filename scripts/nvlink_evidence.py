@@ -73,7 +73,6 @@ def cases():
     if n == 2:
         yield "allreduce_pull_kernel 64MiB", ar(64 * MiB, N.ALGO_PIPE, 3)
         yield "allreduce_pull_kernel 256MiB", ar(256 * MiB, N.ALGO_PIPE, 3)
-        yield "allreduce_push_kernel 64MiB", ar(64 * MiB, N.ALGO_PIPE, 0)
     else:
         if g.has_multicast:
             yield "allreduce_pipe_kernel<NVLS> 256MiB", ar(256 * MiB, N.ALGO_PIPE, 1)

@@ -1,11 +1,11 @@
 """Round-2 tuning sweeps (one process, one rank per GPU, CUDA-graph replay, device-timed).
 
-    python scripts/r02_tune.py --world 2 --what allreduce,sendrecv,gradlocal [--quick]
+    python scripts/r02_tune.py --world 2 --what allreduce,sendrecv,allgather [--quick]
 
 allreduce : phase-by-phase kernels vs the chunk-pipelined ones (allreduce_pipe.cu) over
             chunk size / copy CTAs / reduce CTAs, on ordinary tensors
 sendrecv  : ld/st p2p kernel vs the TMA bulk-copy kernel
-gradlocal : world-1 gradient kernel, units per thread (run with --world 1)
+allgather : staged all-gather vs the pull kernel over copy / pull CTAs
 Output: one line per measurement; the chosen defaults are recorded in profiles/r02/.
 """
 import argparse
@@ -46,7 +46,7 @@ def allreduce(g, args):
             set_all(g, N.PARAM_PIPE_MIN_BYTES, 1 << 40)  # AUTO without the pipeline = round-1 behaviour
             run("staged auto (r01 path)", N.ALGO_AUTO)
             set_all(g, N.PARAM_PIPE_MIN_BYTES, -1)
-            variants = [("pull", 3)] + ([("push", 0)] if args.push else []) if n == 2 else []
+            variants = [("pull", 3)] if n == 2 else []
             if g.has_multicast and n > 2:
                 variants.append(("nvls", 1))
             if args.peer:
@@ -55,11 +55,9 @@ def allreduce(g, args):
                 set_all(g, N.PARAM_PIPE_VARIANT, v)
                 if vname == "pull":
                     grid = [(1, 16, 16), (1, 16, 24), (1, 16, 32), (1, 16, 48), (1, 16, 64), (1, 32, 32), (1, 32, 48), (2, 16, 32)]
-                elif vname == "push":
-                    grid = [(1, 16, 48), (1, 16, 64), (1, 16, 96), (1, 16, 128), (1, 8, 64), (2, 16, 64), (2, 16, 96), (4, 16, 96)]
                 else:
                     grid = [(1, 16, 64), (2, 16, 64), (4, 16, 64), (4, 16, 32), (4, 8, 64), (4, 16, 96), (8, 16, 64), (8, 16, 32)]
-                if args.quick and vname != 'push':
+                if args.quick:
                     grid = grid[1:4]
                 for chunk_mib, copy, red in grid:
                     set_all(g, N.PARAM_PIPE_CHUNK_BYTES, chunk_mib * MiB)
@@ -79,14 +77,12 @@ def sendrecv(g, args):
         xs = [torch.ones(size // 4, device=g.device(r)) for r in range(n)]
         iters = 20 if size <= 64 * MiB else 6
         call = lambda c, r: (c.send(xs[0], 1) if r == 0 else (c.recv(xs[1], 0) if r == 1 else None))  # noqa: E731
-        for label, v, cfg in (("ld/st", 0, -1), ("bulk", -1, -1)):
+        for label, v in (("ld/st", 0), ("bulk", -1)):
             set_all(g, N.PARAM_P2P_BULK_MIN_CHUNK, v)
-            set_all(g, N.PARAM_BULK_CFG, cfg)
             us = time_graphs(g, call, iters)
             print(f"sendrecv n={n} {size / MiB:8.2f} MiB {label:16s} {us:9.1f} us  {size / us / 1e3:7.1f} GB/s", flush=True)
         del xs
     set_all(g, N.PARAM_P2P_BULK_MIN_CHUNK, -1)
-    set_all(g, N.PARAM_BULK_CFG, -1)
 
 
 def allgather(g, args):
@@ -111,45 +107,17 @@ def allgather(g, args):
         set_all(g, p, -1)
 
 
-def gradlocal(g, args):
-    # ResNet-50 DDP buckets (fp32 elements): 7.82, 30.04, 25.04, 25.32, 9.27 MB
-    for mb in (7.82, 9.27, 25.04, 30.04, 60.0, 240.0):
-        numel = int(mb * 1e6 / 4)
-        x = torch.randn(numel, device=g.device(0))
-        flush = torch.empty(256 * MiB // 4, device=g.device(0))
-        for wire in (torch.bfloat16, torch.float32):
-            for unr in (1, 2, 4, 8):
-                set_all(g, N.PARAM_GRAD_LOCAL_UNROLL, unr)
-                c = g.comms[0]
-                times = []
-                for _ in range(12):
-                    flush.zero_()  # evict the bucket from the 126 MB L2
-                    t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                    t0.record()
-                    c.grad_allreduce(x, 0.5, wire)
-                    t1.record()
-                    torch.cuda.synchronize()
-                    times.append(t0.elapsed_time(t1) * 1e3)
-                times = sorted(times[2:])
-                us = times[len(times) // 2]
-                print(f"gradlocal {mb:7.2f} MB wire={str(wire)[6:]:9s} unroll={unr}  {us:8.2f} us  {numel * 8 / us / 1e3:7.1f} GB/s "
-                      f"(min {times[0]:.2f} us)", flush=True)
-        del x, flush
-    set_all(g, N.PARAM_GRAD_LOCAL_UNROLL, -1)
-
-
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--world", type=int, default=2)
     ap.add_argument("--what", default="allreduce,sendrecv")
     ap.add_argument("--quick", action="store_true")
     ap.add_argument("--peer", action="store_true", help="also sweep the peer ld/st pipeline")
-    ap.add_argument("--push", action="store_true", help="also sweep the 2-rank push kernel")
     args = ap.parse_args()
     g = LocalGroup(args.world, timeout_ms=20000, staging_bytes=256 << 20, inbox_bytes=32 << 20)
     print(f"# world={args.world} devices={g.devices} shared={g.shared_gpu} multicast={g.has_multicast}", flush=True)
     for what in args.what.split(","):
-        {"allreduce": allreduce, "sendrecv": sendrecv, "gradlocal": gradlocal, "allgather": allgather}[what](g, args)
+        {"allreduce": allreduce, "sendrecv": sendrecv, "allgather": allgather}[what](g, args)
     g.destroy()
 
 

@@ -1,6 +1,6 @@
 """Timeline of one pipelined all-reduce launch from the in-kernel event trace.
 
-    python scripts/trace_pipe.py --world 2 --variant push --mib 64
+    python scripts/trace_pipe.py --world 2 --variant pull --mib 64
 """
 import argparse
 import os
@@ -15,14 +15,14 @@ from ray_b200.testing import LocalGroup
 
 ap = argparse.ArgumentParser()
 ap.add_argument("--world", type=int, default=2)
-ap.add_argument("--variant", default="push")
+ap.add_argument("--variant", default="pull")
 ap.add_argument("--mib", type=int, default=64)
 ap.add_argument("--copy", type=int, default=-1)
 ap.add_argument("--red", type=int, default=-1)
 ap.add_argument("--chunk", type=int, default=-1)
 ap.add_argument("--ctas", default="0,1,16,17")
 args = ap.parse_args()
-V = {"push": 0, "nvls": 1, "peer": 2, "pull": 3}[args.variant]
+V = {"nvls": 1, "peer": 2, "pull": 3}[args.variant]
 g = LocalGroup(args.world, timeout_ms=10000, staging_bytes=256 << 20, inbox_bytes=8 << 20)
 for c in g.comms:
     c.set_param(N.PARAM_PIPE_VARIANT, V)
@@ -43,7 +43,7 @@ by_cta = defaultdict(list)
 for ns, cta, e, a in ev:
     by_cta[cta].append(((ns - t0) / 1e3, e, a))
 names = {1: "load", 2: "store", 3: "ringok", 4: "done<", 5: "drain", 6: "gateok", 9: "flag:see", 10: "flag:proxyfenced", 13: "flag:sysfenced", 11: "flag:arrived", 12: "flag:signal",
-         30: "pl:load", 31: "pl:gatewait", 32: "pl:gateok", 33: "pl:landed", 20: "red:wait", 21: "red:go", 22: "red:itemend", 23: "red:arrived", 41: "o:load", 42: "o:store", 43: "o:ringok", 44: "o:done<",
+         30: "pl:load", 31: "pl:gatewait", 32: "pl:gateok", 33: "pl:landed", 23: "red:arrived", 41: "o:load", 42: "o:store", 43: "o:ringok", 44: "o:done<",
          45: "o:drain", 46: "o:gateok"}
 for cta in [int(x) for x in args.ctas.split(",")]:
     rows = by_cta.get(cta, [])

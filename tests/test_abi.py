@@ -24,6 +24,26 @@ def test_header_declares_what_the_binding_binds():
     assert sorted(_native.SIGNATURES) == declared
 
 
+def _declared_enumerators(typedef):
+    text = re.sub(r"/\*.*?\*/", "", open(HEADER).read(), flags=re.S)
+    body = re.search(r"typedef enum \{([^}]*)\}\s*" + typedef + r";", text)
+    assert body, f"enum {typedef} not found in the header"
+    return {name: int(value) for name, value in re.findall(r"\b(B200_\w+)\s*=\s*(-?\d+)", body.group(1))}
+
+
+def test_header_enums_match_the_binding_constants():
+    """Parameter and algorithm numbers are part of the ABI: the binding's PARAM_* / ALGO_* must be
+    exactly the header's enumerators, value for value."""
+    for typedef, prefix, count in (("b200_param_t", "PARAM_", "B200_PARAM_COUNT"), ("b200_algo_t", "ALGO_", None)):
+        declared = _declared_enumerators(typedef)
+        assert declared, typedef
+        if count:
+            assert declared.pop(count) == len(declared), f"{count} is not the number of parameters"
+            assert sorted(declared.values()) == list(range(len(declared))), f"{typedef} is not contiguous"
+        bound = {f"B200_{k}": v for k, v in vars(_native).items() if k.startswith(prefix)}
+        assert bound == declared, typedef
+
+
 def test_library_exports_every_declared_symbol(native_lib):
     out = subprocess.run(["nm", "-D", "--defined-only", str(_native.LIB_PATH)], capture_output=True, text=True,
                          check=True).stdout

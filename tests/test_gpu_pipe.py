@@ -1,7 +1,7 @@
 """GPU parity tests of the chunk-pipelined all-reduce kernels (allreduce_pipe.cu: TMA bulk-copy
 roles + reduce role synchronised by per-chunk flags) against the rank-ascending oracle.
 
-Peer ld/st and push variants are bit exact against the oracle for every dtype; the NVLS variant
+Peer ld/st and pull variants are bit exact against the oracle for every dtype; the NVLS variant
 (multi-GPU boxes only) is exact on integer-valued data and within 1e-6 * sum|x| otherwise.
 """
 import numpy as np
@@ -39,7 +39,7 @@ def _variants(g, world):
 
     out = [("peer", 2)]
     if world == 2:
-        out += [("pull", 3), ("push", 0)]
+        out.append(("pull", 3))
     if g.has_multicast:
         out.append(("nvls", 1))
     return out, N
@@ -290,29 +290,47 @@ def test_pull_allgather_is_byte_exact(pipe_groups, world):
 @pytest.mark.parametrize("world", [3, 4])
 def test_chunk_ring_handles_messages_larger_than_the_staging_slot_in_one_launch(pipe_groups, world):
     """n >= 3 pipeline with the slot used as a ring of chunks: a message several times the slot
-    size goes through ONE launch (copy-in of chunk k waits for the copy-out of chunk k - R);
-    B200_PARAM_PIPE_RING=0 splits it into several launches and must give the same bits."""
+    size goes through ONE launch (copy-in of chunk k waits for the copy-out of chunk k - R).  A
+    chunk size that leaves fewer than 4 chunks in the slot turns the ring off, and the message is
+    split into launches of as many whole chunks as the slot holds; that must give the same bits."""
     from ray_b200 import _native as N
 
-    g = pipe_groups(world)  # 40 MiB staging slot
-    numel = (97 * MiB + 16 * 3) // 4
+    staging = 40 * MiB
+    g = pipe_groups(world)
+    nbytes = 97 * MiB + 16 * 3
+    numel = nbytes // 4
     host = [(torch.arange(numel, dtype=torch.float32) % 1021) * (r + 1) - 3 * r for r in range(world)]
     want = sum(host)
     try:
-        for chunk in (1 * MiB, 4 * MiB):
-            for ring in (-1, 0):
-                for c in g.comms:
-                    c.set_param(N.PARAM_PIPE_CHUNK_BYTES, chunk)
-                    c.set_param(N.PARAM_PIPE_RING, ring)
-                xs = [h.to(g.device(r)) for r, h in enumerate(host)]
-                before = g.comms[0].launch_count
-                g.run(lambda c, r: c.allreduce(xs[r], N.SUM, algo=N.ALGO_PIPE))
-                launches = g.comms[0].launch_count - before
-                assert launches == (1 if ring == -1 else 3), (chunk, ring, launches)
-                for r in range(world):
-                    assert torch.equal(xs[r].cpu(), want), (world, chunk, ring, r)
-                del xs
+        for chunk in (1 * MiB, 4 * MiB, 16 * MiB):
+            ring = staging // chunk >= 4
+            split = staging // chunk * chunk  # bytes per launch without the ring
+            for c in g.comms:
+                c.set_param(N.PARAM_PIPE_CHUNK_BYTES, chunk)
+            xs = [h.to(g.device(r)) for r, h in enumerate(host)]
+            before = g.comms[0].launch_count
+            g.run(lambda c, r: c.allreduce(xs[r], N.SUM, algo=N.ALGO_PIPE))
+            launches = g.comms[0].launch_count - before
+            assert launches == (1 if ring else -(-nbytes // split)), (chunk, launches)
+            for r in range(world):
+                assert torch.equal(xs[r].cpu(), want), (world, chunk, r)
+            del xs
     finally:
         for c in g.comms:
             c.set_param(N.PARAM_PIPE_CHUNK_BYTES, -1)
-            c.set_param(N.PARAM_PIPE_RING, -1)
+
+
+def test_pipe_variant_parameter_rejects_unknown_values(pipe_groups):
+    """B200_PARAM_PIPE_VARIANT takes -1 (automatic), 1 (NVLS), 2 (peer) or 3 (pull); anything else,
+    such as 0 for the removed push kernel, is refused instead of silently selecting another kernel."""
+    from ray_b200 import _native as N
+
+    c = pipe_groups(2).comms[0]
+    try:
+        for bad in (0, 4, -2):
+            with pytest.raises(N.B200Error):
+                c.set_param(N.PARAM_PIPE_VARIANT, bad)
+        for good in (1, 2, 3, -1):
+            c.set_param(N.PARAM_PIPE_VARIANT, good)
+    finally:
+        c.set_param(N.PARAM_PIPE_VARIANT, -1)
